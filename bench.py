@@ -238,6 +238,23 @@ def parity_rows(m: int):
     return np.sort(rng.choice(m, size=min(PARITY_ROWS, m), replace=False))
 
 
+DUMP_BYTES_MAX, DUMP_SEED = 64 * 10**6, 4321
+
+
+def dump_outputs(out_dir, result) -> None:
+    """--dump-outputs: the fp64 result [m, dv] that rank 0's caller received from the last timed step, as result.npy.  Above
+    DUMP_BYTES_MAX it is a fixed seeded sample of rows (sorted) instead, their indices in result_rows.npy (float64, exact)."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    row_bytes = result.shape[1] * result.itemsize
+    if result.nbytes > DUMP_BYTES_MAX:
+        keep = (DUMP_BYTES_MAX - 4096) // (row_bytes + 8)     # 4096: room for the two .npy headers
+        rows = np.sort(np.random.default_rng(DUMP_SEED).choice(result.shape[0], size=keep, replace=False))
+        np.save(os.path.join(out_dir, "result_rows.npy"), rows.astype(np.float64))
+        result = result[rows]
+    np.save(os.path.join(out_dir, "result.npy"), np.ascontiguousarray(result, dtype=np.float64))
+
+
 def oracle_rows(m: int, shard_rows, rows):
     """fp64 oracle (oracle.attention_f64_numpy = attention.c:20-75) of the selected Q rows against the FULL K/V,
     every shard regenerated from its seed.  Checker only: runs outside every timed region, on rank 0."""
@@ -516,8 +533,9 @@ def run_ours(args) -> None:
             collect(ctx.accumulated_timings(reset=True))
         return parallel.max_over_ranks(e0.elapsed_time(e1))  # ms, max over ranks
 
-    def measure(name, W, K, sampler=None, m_override=0, n_per_gpu_override=0, prec_override=None, parity=True):
-        """Warm-up, K timed device-resident steps, K timed host (e2e) steps, oracle parity check.  Collective over ranks."""
+    def measure(name, W, K, sampler=None, m_override=0, n_per_gpu_override=0, prec_override=None, parity=True, keep_result=False):
+        """Warm-up, K timed device-resident steps, K timed host (e2e) steps, oracle parity check.  Collective over ranks.
+        keep_result: rank 0 also returns (as "result") the fp64 output its last timed device-resident step wrote."""
         cfg = CONFIGS[name]
         prec = prec_override or cfg["prec"]
         m, shard_rows = config_shape(name, world, m_override, n_per_gpu_override)
@@ -527,6 +545,13 @@ def run_ours(args) -> None:
             wl.step_device()
         ctx.synchronize()
         stage = {"ms": 0.0, "launches": 0.0, "cast_ms": 0.0, "merge_ms": 0.0, "total_ms": 0.0, "calls": 0.0}
+        result = []
+
+        def timed_device():
+            ms = timed(ctx, wl.step_device, K, collect)
+            if keep_result and wl.Rd is not None:   # copied before any later step writes the buffer again
+                result.append(wl.Rd.cpu().numpy())
+            return ms
 
         def collect(t):
             stage["ms"] += t["fused_ms"]
@@ -540,7 +565,7 @@ def run_ours(args) -> None:
         launches0 = sdpa_b200.launch_count()
         if sampler is not None:
             with sampler as clk:
-                ms_dev = timed(ctx, wl.step_device, K, collect)
+                ms_dev = timed_device()
                 launches = sdpa_b200.launch_count() - launches0   # kernels launched inside the timed region only
                 # The timed region is a few milliseconds: keep the identical load running so the sampler sees it.
                 # Every step is collective across ranks, so the extra steps are a COUNT derived from the
@@ -552,7 +577,7 @@ def run_ours(args) -> None:
                 barrier()
             clocks = clk.summary()
         else:
-            ms_dev = timed(ctx, wl.step_device, K, collect)
+            ms_dev = timed_device()
             launches = sdpa_b200.launch_count() - launches0
         kernel_name = ctx.last_kernel()
         issue_us = host_enqueue_us[0]
@@ -568,7 +593,7 @@ def run_ours(args) -> None:
             "ms_dev": ms_dev, "ms_host": ms_host, "flops_step": wl.flops_step, "launches": int(launches),
             "value": wl.flops_step * K / (ms_dev * 1e-3) / 1e12, "e2e_value": wl.flops_step * K / (ms_host * 1e-3) / 1e12,
             "h2d": wl.h2d_bytes(), "d2h": wl.d2h_bytes(), "stage": stage, "clocks": clocks, "parity": parity, "host_issue_us": issue_us,
-            "q_batches": -(-m // (args.q_batch or 8192)),
+            "q_batches": -(-m // (args.q_batch or 8192)), "result": result[0] if result else None,
         }
         wl.free()
         ctx.close()
@@ -582,8 +607,10 @@ def run_ours(args) -> None:
     sampler = ClockSampler(local_rank, gpu_uuid, allow_subprocess=(rank == 0)).start()
     barrier()
 
-    W, K = max(3, args.warmup), max(1, args.steps)
-    head = measure(args.config, W, K, sampler, args.m, args.n_per_gpu, args.precision)
+    W, K = max(3, args.warmup), args.steps
+    head = measure(args.config, W, K, sampler, args.m, args.n_per_gpu, args.precision, keep_result=bool(args.dump_outputs))
+    if rank == 0 and args.dump_outputs:
+        dump_outputs(args.dump_outputs, head["result"])
     clocks = head["clocks"]
     sampler.close()
     if world > 1:   # every rank sampled its own GPU: report the slowest median clock and the union of the reasons
@@ -606,7 +633,7 @@ def run_ours(args) -> None:
     extra_errors = {}
     for name in extra_names:
         try:
-            r = measure(name, 3, max(3, min(K, 10)))
+            r = measure(name, 3, K)
         except Exception as exc:   # an extra configuration must not cost the headline line; the failure is reported in it
             extra_errors[name] = repr(exc)
             print("bench: extra configuration %s failed: %r" % (name, exc), file=sys.stderr)
@@ -776,7 +803,14 @@ def main() -> None:
     ap.add_argument("--stage-timing-every", type=int, default=4,
                     help="stage marks (CUDA events around cast / fused kernel / merge) on every k-th queued pass (1 = every pass)")
     ap.add_argument("--no-cpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default="",
+                    help="after the timed steps, write the output of the headline's last timed step to DIR/result.npy (fp64; inputs are "
+                         "seeded, so runs with the same arguments compare output for output)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the GPU path's output: it needs --impl ours")
     if args.impl == "reference":
         run_reference_arm(args)
     else:

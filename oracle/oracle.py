@@ -39,8 +39,9 @@ _c_double_p = ctypes.POINTER(ctypes.c_double)
 _c_float_p = ctypes.POINTER(ctypes.c_float)
 
 
-def build(reference: str | os.PathLike | None = "/root/reference", quiet: bool = True) -> None:
-    """Compile the C restatement and, if the reference sources are present, oracle/_ref."""
+def build(reference: str | os.PathLike | None = None, quiet: bool = True) -> None:
+    """Compile the C restatement and, if the reference sources are present, oracle/_ref.  reference=None: the
+    Makefile's default (REFERENCE from the environment, else the checkout next to this repository)."""
     args = ["make", "-C", str(HERE), "all"]
     if reference is not None:
         args.append(f"REFERENCE={reference}")

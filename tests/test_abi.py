@@ -1,6 +1,9 @@
 """The C-ABI library loads without a GPU and exports every symbol include/sdpa_b200.h declares."""
 import ctypes
+import os
 import re
+import subprocess
+import sys
 from pathlib import Path
 
 import pytest
@@ -43,11 +46,16 @@ def test_owner_map_matches_reference_formula(sdpa, oracle):
 
 
 def test_no_cpu_fallback(sdpa):
-    """Without a CUDA device the engine refuses to create a context (and says why)."""
-    if sdpa.device_count() > 0:
-        pytest.skip("GPU present")
-    with pytest.raises(sdpa.SdpaError, match="no CPU fallback"):
-        sdpa.Context()
+    """Without a CUDA device the engine refuses to create a context (and says why).  Where a GPU is present, a child
+    process with every device hidden makes the same attempt."""
+    if sdpa.device_count() == 0:
+        with pytest.raises(sdpa.SdpaError, match="no CPU fallback"):
+            sdpa.Context()
+        return
+    code = ("import sdpa_b200\ntry:\n    sdpa_b200.Context()\nexcept sdpa_b200.SdpaError as e:\n    print('refused:', e)\n")
+    r = subprocess.run([sys.executable, "-c", code], capture_output=True, text=True, timeout=300, cwd=str(ROOT),
+                       env={**os.environ, "CUDA_VISIBLE_DEVICES": ""})
+    assert r.returncode == 0 and "refused:" in r.stdout and "no CPU fallback" in r.stdout, r
 
 
 def test_version_string(sdpa):

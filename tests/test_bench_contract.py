@@ -1,6 +1,7 @@
-"""bench.py contract checks that need no GPU: the reference arm prints one JSON line with the keys
-the driver reads (it runs the reference's own CPU program -- oracle/_ref -- or the oracle port)."""
+"""bench.py contract checks, all but the last --dump-outputs one without a GPU: the reference arm prints one JSON line with
+the keys the driver reads (it runs the reference's own CPU program -- oracle/_ref -- or the oracle port)."""
 import json
+import os
 import subprocess
 import sys
 from pathlib import Path
@@ -28,9 +29,9 @@ def test_reference_arm_json_line(oracle):
 
 
 def test_our_arm_refuses_without_gpu(sdpa):
-    if sdpa.device_count() > 0:
-        pytest.skip("GPU present")
-    r = subprocess.run([sys.executable, str(ROOT / "bench.py"), "--steps", "1"], capture_output=True, text=True, timeout=300, cwd=str(ROOT))
+    """Every device is hidden from the child, so this runs the same on a GPU machine."""
+    r = subprocess.run([sys.executable, str(ROOT / "bench.py"), "--steps", "1"], capture_output=True, text=True, timeout=300, cwd=str(ROOT),
+                       env={**os.environ, "CUDA_VISIBLE_DEVICES": ""})
     assert r.returncode != 0 and "no CPU fallback" in (r.stderr + r.stdout)
 
 
@@ -50,6 +51,54 @@ def test_clock_sampler_summary_and_graceful_start():
         pass
     live.close()
     assert live.summary()["samples"] >= 0
+
+
+def test_steps_must_be_positive():
+    r = subprocess.run([sys.executable, str(ROOT / "bench.py"), "--steps", "0"], capture_output=True, text=True, timeout=300, cwd=str(ROOT))
+    assert r.returncode == 2 and "--steps must be at least 1" in r.stderr
+
+
+def test_dump_outputs_writes_the_result_or_a_seeded_row_sample(tmp_path, monkeypatch):
+    sys.path.insert(0, str(ROOT))
+    import numpy as np
+    import bench
+    res = np.random.default_rng(0).standard_normal((300, 128))
+    bench.dump_outputs(str(tmp_path / "all"), res)
+    assert sorted(p.name for p in (tmp_path / "all").iterdir()) == ["result.npy"]
+    assert np.array_equal(np.load(tmp_path / "all" / "result.npy"), res)
+    monkeypatch.setattr(bench, "DUMP_BYTES_MAX", 100 * 128 * 8)       # room for fewer than 100 of the 300 rows
+    for d in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / d), res)
+    got, rows = np.load(tmp_path / "a" / "result.npy"), np.load(tmp_path / "a" / "result_rows.npy")
+    assert got.dtype == np.float64 and rows.dtype == np.float64
+    assert got.nbytes + rows.nbytes <= bench.DUMP_BYTES_MAX and 0 < len(rows) < 100
+    assert np.all(np.diff(rows) > 0) and np.array_equal(got, res[rows.astype(np.int64)])
+    assert np.array_equal(rows, np.load(tmp_path / "b" / "result_rows.npy"))      # the same sample every run
+
+
+@pytest.mark.gpu
+@pytest.mark.timeout(900)
+def test_dump_outputs_is_the_timed_result(oracle, tmp_path):
+    """--dump-outputs writes what the last timed step returned: the full [m, dv] fp64 result, within the bf16 path's tolerance
+    of the fp64 oracle on the parity rows.  --steps sets the passes the timed region runs: with stage marks on every pass, the
+    library's count of marked passes between the two reads around the timed loop is --steps."""
+    import numpy as np
+    sys.path.insert(0, str(ROOT))
+    import bench
+    m, n = 512, 4096
+    r = subprocess.run([sys.executable, str(ROOT / "bench.py"), "--gpus", "1", "--steps", "3", "--warmup", "1", "--m", str(m),
+                        "--n-per-gpu", str(n), "--extra", "none", "--no-alone", "--no-cpu-baseline", "--stage-timing-every", "1",
+                        "--dump-outputs", str(tmp_path)],
+                       capture_output=True, text=True, timeout=880, cwd=str(ROOT))
+    assert r.returncode == 0, r.stderr[-2000:]
+    line = json.loads([l for l in r.stdout.splitlines() if l.startswith("{")][-1])
+    assert line["steps"] == 3 and line["stage_ms_per_step"]["passes_timed"] == 3
+    assert line["config"]["m"] == m and line["config"]["n"] == n
+    assert sorted(p.name for p in tmp_path.iterdir()) == ["result.npy"]
+    got = np.load(tmp_path / "result.npy")
+    assert got.shape == (m, bench.DV) and got.dtype == np.float64
+    rows = bench.parity_rows(m)
+    np.testing.assert_allclose(got[rows], bench.oracle_rows(m, [n], rows), rtol=0, atol=bench.CONFIGS["c3"]["tol"])
 
 
 def test_bench_config_shapes_match_baseline():
