@@ -37,13 +37,21 @@ typedef enum sdpa_status {
 /* Arithmetic of the fused QK^T -> softmax -> .V kernel. */
 typedef enum sdpa_precision {
     SDPA_PREC_AUTO = 0,  /* fp32-class accuracy, like the reference (mpi.c:168-189): BF16X3 where that kernel takes the shape,
-                            else F32.  Never BF16: the reference's 0.02 gate (mpi.c:476) must hold on peaky inputs           */
+                            else F32.  Never BF16 for fp64 / fp32 operands: the reference's 0.02 gate (mpi.c:476) must hold on
+                            peaky inputs.  bf16 operands (typed passes): BF16 where it takes the shape, else F32           */
     SDPA_PREC_F32 = 1,   /* fp32 CUDA-core kernel: the reference's own arithmetic; any dk, dv <= 256                        */
     SDPA_PREC_BF16 = 2,  /* opt-in: bf16 operands, fp32 accumulate, tcgen05; dk, dv multiples of 8 up to 256                */
     SDPA_PREC_BF16X3 = 3 /* fp32 operands split into bf16 hi + lo, three tcgen05.mma per contraction into one fp32
                             accumulator (<= 1e-5 on N(0,1) inputs); dk, dv multiples of 8 with dk <= 128 and dv <= 128, or
                             dk <= 64 and dv <= 256 (what fits the 227 KiB of shared memory)                                */
 } sdpa_precision;
+
+/* Element type of the device arrays of a typed pass (sdpa_attention_device_typed); the result has the same type. */
+typedef enum sdpa_dtype {
+    SDPA_DTYPE_F64 = 0,  /* the reference's own operands: the same pass as sdpa_attention_device_full                         */
+    SDPA_DTYPE_F32 = 1,
+    SDPA_DTYPE_BF16 = 2  /* raw bfloat16 (1 sign, 8 exponent, 7 mantissa bits), e.g. torch.bfloat16                            */
+} sdpa_dtype;
 
 /* How the per-shard softmax states are merged across GPUs (mpi.c:340-380). */
 typedef enum sdpa_merge {
@@ -80,6 +88,11 @@ typedef struct sdpa_ctx sdpa_ctx;
 /* Whether a kernel exists for (precision, dk, dv); for SDPA_PREC_AUTO always 1 when dk, dv are in [1, 256], and
  * *resolved (may be NULL) receives the precision AUTO selects.  Pure host function; usable without a GPU. */
 int sdpa_precision_supported(int precision, int dk, int dv, int* resolved);
+/* The same for operands of element type `dtype` (sdpa_dtype).  fp64 and fp32 operands: the rule above.  bf16 operands: AUTO
+ * resolves to BF16 where the bf16 tensor-core kernel takes (dk, dv), else F32 -- the operands are already rounded to bf16 by
+ * the caller, so the operand rounding that keeps plain bf16 out of AUTO for fp64 / fp32 operands does not arise; what remains
+ * is the bf16 rounding of the softmax weights P (<= 2e-3 on N(0,1) inputs).  Pure host function; usable without a GPU. */
+int sdpa_precision_supported_for(int dtype, int precision, int dk, int dv, int* resolved);
 
 /* ---------------------------------------------------------------------------
  * 1. The reference entry point (replaces mpi.c:191-192; the serial flavour
@@ -181,6 +194,20 @@ sdpa_status sdpa_enqueue_device_full(sdpa_ctx* ctx, const double* const* K_shard
  * kernel variant; blocking calls carry that variant in the stream instead), so results are final on return -- which is why the
  * arrays of queued passes must stay valid until then.  On a context that spans several processes the call is collective. */
 sdpa_status sdpa_synchronize(sdpa_ctx* ctx);
+
+/* sdpa_attention_device_full / sdpa_enqueue_device_full on device arrays of element type `dtype` (sdpa_dtype): K/V shards,
+ * Q and the result are dense row-major arrays of that type, the result (m x dv, root process only) too.  SDPA_DTYPE_F64 is
+ * exactly the fp64 call.  The kernel follows sdpa_precision_supported_for(dtype, cfg.precision, dk, dv).  No fp64 copy is
+ * made: the casts into compute precision read the caller's arrays, and where the arrays already are in compute precision
+ * (bf16 operands at BF16, fp32 operands at F32) the fused kernel reads them in place and no cast runs at all -- which for the
+ * tensor-core kernels needs K, V and Q 16-byte aligned (else SDPA_ERR_INVALID; nothing is copied to make up for it).  The
+ * result is merged in fp64 and rounded once (round to nearest even) into `dtype`.  The queued form has the contract of
+ * sdpa_enqueue_device_full: arrays valid and unmodified until sdpa_synchronize(), which also repairs its passes.  Typed
+ * passes never cast ahead. */
+sdpa_status sdpa_attention_device_typed(sdpa_ctx* ctx, int dtype, const void* const* K_shards, const void* const* V_shards,
+                                        const int* n_local, int dk, int dv, const void* const* Q_dev, void* result_dev, int m);
+sdpa_status sdpa_enqueue_device_typed(sdpa_ctx* ctx, int dtype, const void* const* K_shards, const void* const* V_shards,
+                                      const int* n_local, int dk, int dv, const void* const* Q_dev, void* result_dev, int m);
 
 /* The reference's calling convention on a one-GPU-per-process context (world_size > 1):
  * dimensions and Q/K/V/result are valid on the process that owns shard 0 only; that process

@@ -891,6 +891,7 @@ struct UmmaPlan {
     const void* k_base = nullptr;
     const void* v_base = nullptr;
     int q_rows[2] = {0, 0};
+    size_t q_lo[2] = {0, 0};
     bool attr_set[64] = {};
     // Overflow guard: a ring of kGuardRing device words; the launch with epoch e uses word e % kGuardRing and a fast kernel writes
     // e into it when an exponent would overflow.  A word equals a launch's epoch only if THAT launch raised it, so the words are
@@ -980,7 +981,7 @@ sdpa_status umma_plan_bind_q(UmmaPlan* plan, int slot, const __nv_bfloat16* Q, i
         set_error("umma_plan_bind_q: bad slot, or dk / precision differ from the bound K/V shard");
         return SDPA_ERR_INVALID;
     }
-    if (plan->q_bound[slot] && plan->q_base[slot] == Q && plan->q_rows[slot] == rows_capacity) return SDPA_OK;
+    if (plan->q_bound[slot] && plan->q_base[slot] == Q && plan->q_rows[slot] == rows_capacity && plan->q_lo[slot] == q_lo_off) return SDPA_OK;
     {
         SDPA_TRY(encode_map(&plan->gmaps[slot][0], Q, rows_capacity, TILE, dk));
         SDPA_TRY(encode_map(&plan->gmaps[slot][1], Q + (hl == 2 ? q_lo_off : 0), rows_capacity, TILE, dk));
@@ -989,6 +990,7 @@ sdpa_status umma_plan_bind_q(UmmaPlan* plan, int slot, const __nv_bfloat16* Q, i
     plan->q_bound[slot] = true;
     plan->q_base[slot] = Q;
     plan->q_rows[slot] = rows_capacity;
+    plan->q_lo[slot] = q_lo_off;
     return SDPA_OK;
 }
 

@@ -131,13 +131,17 @@ cvt_d2bf16_scalar_kernel(__nv_bfloat16* __restrict__ dst, const double* __restri
         dst[i] = __float2bfloat16_rn(__double2float_rn(src[i]));
 }
 
-// fp64 -> (hi, lo) bf16 pair of the split precision: x32 = fp32(x) (the reference's own cvt_d2f, mpi.c:31-64), hi = bf16(x32),
-// lo = bf16(x32 - hi): hi + lo carries 16 mantissa bits of x32.  12 B per element like d2f (8 read, 2 + 2 written).
-__device__ __forceinline__ void split_bf16x2(double2 v, uint32_t& hi, uint32_t& lo)
+// fp32 pair -> (hi, lo) bf16 pairs of the split precision: hi = bf16(x32), lo = bf16(x32 - hi): hi + lo carries 16 mantissa
+// bits of x32.  For a bf16 x32, hi = x32 and lo = 0.
+__device__ __forceinline__ void split_bf16x2(float a, float b, uint32_t& hi, uint32_t& lo)
 {
-    const float a = __double2float_rn(v.x), b = __double2float_rn(v.y);
     hi = pack_bf16x2(a, b);
     lo = pack_bf16x2(a - __uint_as_float(hi << 16), b - __uint_as_float(hi & 0xffff0000u));
+}
+// fp64 -> (hi, lo): x32 = fp32(x) (the reference's own cvt_d2f, mpi.c:31-64) first.  12 B per element like d2f (8 read, 2 + 2 written).
+__device__ __forceinline__ void split_bf16x2(double2 v, uint32_t& hi, uint32_t& lo)
+{
+    split_bf16x2(__double2float_rn(v.x), __double2float_rn(v.y), hi, lo);
 }
 
 __global__ void __launch_bounds__(kCastThreads)
@@ -178,54 +182,107 @@ cvt_d2bf16x2_scalar_kernel(__nv_bfloat16* __restrict__ dst_hi, __nv_bfloat16* __
     }
 }
 
-// Several fp64 -> compute-precision casts in ONE launch (the K shard, the V shard and the first Q batch of a
-// device-resident call): the segments form one virtual array of 2-element units, so the grid-stride loop has a
-// single tail instead of one per operand and two launch gaps disappear from the step.
-// MODE 0: fp32, 1: bf16, 2: bf16 hi/lo split (lo array cb.lo_off[seg] 2-element units behind the hi array)
-template <int MODE>
+// Source element types of the batched cast: fp64 (the reference's operands) and, for typed device passes, fp32 and bf16.
+// Unit = 2 elements, loaded as one vector and widened to an fp32 pair (fp64 rounds to nearest even, like cvt_d2f; fp32 and
+// bf16 are exact).
+template <typename SRC> struct SrcPair;
+template <> struct SrcPair<double> {
+    using Unit = double2;
+    static __device__ __forceinline__ Unit load(const Unit* p) { return ld_stream_f64x2(p); }
+    static __device__ __forceinline__ float2 f32(Unit v) { return make_float2(__double2float_rn(v.x), __double2float_rn(v.y)); }
+};
+template <> struct SrcPair<float> {
+    using Unit = float2;
+    static __device__ __forceinline__ Unit load(const Unit* p)
+    {
+        float2 v;
+        asm volatile("ld.global.nc.L1::no_allocate.v2.f32 {%0, %1}, [%2];" : "=f"(v.x), "=f"(v.y) : "l"(p));
+        return v;
+    }
+    static __device__ __forceinline__ float2 f32(Unit v) { return v; }
+};
+template <> struct SrcPair<__nv_bfloat16> {
+    using Unit = uint32_t;   // two bf16, the first in the low half
+    static __device__ __forceinline__ Unit load(const Unit* p)
+    {
+        uint32_t v;
+        asm volatile("ld.global.nc.L1::no_allocate.b32 %0, [%1];" : "=r"(v) : "l"(p));
+        return v;
+    }
+    static __device__ __forceinline__ float2 f32(Unit v) { return make_float2(__uint_as_float(v << 16), __uint_as_float(v & 0xffff0000u)); }
+};
+
+// Several casts into compute precision in ONE launch (the K shard, the V shard and the first Q batch of a device-resident
+// call): the segments form one virtual array of 2-element units, so the grid-stride loop has a single tail instead of one
+// per operand and two launch gaps disappear from the step.
+// MODE 0: fp32, 1: bf16, 2: bf16 hi/lo split (lo array cb.lo_off[seg] 2-element units behind the hi array).  Every mode
+// goes through the fp32 pair of SrcPair<SRC>, so an fp32 source gives the bits an fp64 source of the same fp32 values gives.
+template <typename SRC, int MODE>
 __global__ void __launch_bounds__(kCastThreads) cvt_in_batch_kernel(CastBatch cb)
 {
+    using P = SrcPair<SRC>;
+    using Unit = typename P::Unit;
     const size_t u0 = cb.units[0], u01 = u0 + cb.units[1], all = u01 + cb.units[2];
     const size_t total = (size_t)gridDim.x * blockDim.x;
-    auto locate = [&](size_t g, const double2*& src, void*& dst, size_t& off, size_t& lo) {
+    auto locate = [&](size_t g, const Unit*& src, void*& dst, size_t& off, size_t& lo) {
         const int seg = g < u0 ? 0 : (g < u01 ? 1 : 2);
         off = g - (seg == 0 ? 0 : (seg == 1 ? u0 : u01));
-        src = reinterpret_cast<const double2*>(cb.src[seg]);
+        src = reinterpret_cast<const Unit*>(cb.src[seg]);
         dst = cb.dst[seg];
         lo = cb.lo_off[seg];
     };
-    auto store = [&](void* dst, size_t off, size_t lo, double2 v) {
+    auto store = [&](void* dst, size_t off, size_t lo, Unit u) {
+        const float2 v = P::f32(u);
         if (MODE == 2) {
             uint32_t h, l;
-            split_bf16x2(v, h, l);
+            split_bf16x2(v.x, v.y, h, l);
             reinterpret_cast<uint32_t*>(dst)[off] = h;
             reinterpret_cast<uint32_t*>(dst)[off + lo] = l;
         } else if (MODE == 1) {
-            reinterpret_cast<uint32_t*>(dst)[off] = pack_bf16x2(__double2float_rn(v.x), __double2float_rn(v.y));
+            reinterpret_cast<uint32_t*>(dst)[off] = pack_bf16x2(v.x, v.y);
         } else {
-            reinterpret_cast<float2*>(dst)[off] = make_float2(__double2float_rn(v.x), __double2float_rn(v.y));
+            reinterpret_cast<float2*>(dst)[off] = v;
         }
     };
     size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
     for (; i + (kUnroll - 1) * total < all; i += kUnroll * total) {
-        double2 v[kUnroll];
+        Unit v[kUnroll];
         void* d[kUnroll];
         size_t off[kUnroll], lo[kUnroll];
 #pragma unroll
         for (int u = 0; u < kUnroll; ++u) {
-            const double2* src;
+            const Unit* src;
             locate(i + u * total, src, d[u], off[u], lo[u]);
-            v[u] = ld_stream_f64x2(src + off[u]);
+            v[u] = P::load(src + off[u]);
         }
 #pragma unroll
         for (int u = 0; u < kUnroll; ++u) store(d[u], off[u], lo[u], v[u]);
     }
     for (; i < all; i += total) {
-        const double2* src;
+        const Unit* src;
         void* d;
         size_t off, lo;
         locate(i, src, d, off, lo);
-        store(d, off, lo, ld_stream_f64x2(src + off));
+        store(d, off, lo, P::load(src + off));
+    }
+}
+
+// Scalar form of one fp32 / bf16 segment (unaligned pointers, odd counts): the same conversions, one element per thread.
+template <typename SRC, int MODE>
+__global__ void __launch_bounds__(kCastThreads)
+cvt_typed_scalar_kernel(void* __restrict__ dst, size_t lo_off, const SRC* __restrict__ src, size_t count)
+{
+    const size_t stride = (size_t)gridDim.x * blockDim.x;
+    for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < count; i += stride) {
+        const float a = (float)src[i];
+        if (MODE == 0) {
+            reinterpret_cast<float*>(dst)[i] = a;
+        } else {
+            __nv_bfloat16* d = reinterpret_cast<__nv_bfloat16*>(dst);
+            const __nv_bfloat16 h = __float2bfloat16_rn(a);
+            d[i] = h;
+            if (MODE == 2) d[i + lo_off] = __float2bfloat16_rn(a - __bfloat162float(h));
+        }
     }
 }
 
@@ -382,9 +439,9 @@ sdpa_status launch_stamp(unsigned long long* dst, cudaStream_t stream)
 void preload_cast_kernels()
 {
     cudaFuncAttributes a;
-    cudaFuncGetAttributes(&a, cvt_in_batch_kernel<0>);
-    cudaFuncGetAttributes(&a, cvt_in_batch_kernel<1>);
-    cudaFuncGetAttributes(&a, cvt_in_batch_kernel<2>);
+    cudaFuncGetAttributes(&a, cvt_in_batch_kernel<double, 0>);
+    cudaFuncGetAttributes(&a, cvt_in_batch_kernel<double, 1>);
+    cudaFuncGetAttributes(&a, cvt_in_batch_kernel<double, 2>);
     cudaFuncGetAttributes(&a, cvt_in_batch_bg_kernel<0>);
     cudaFuncGetAttributes(&a, cvt_in_batch_bg_kernel<1>);
     cudaFuncGetAttributes(&a, cvt_in_batch_bg_kernel<2>);
@@ -471,15 +528,40 @@ sdpa_status launch_cvt_d2bf16x2(__nv_bfloat16* dst_hi, __nv_bfloat16* dst_lo, co
     return SDPA_OK;
 }
 
-// Up to three operands in one launch; falls back to one launch per operand when a pointer is not 16-byte aligned
-// or a count is odd (the batched kernel moves 2-element units only).
-sdpa_status launch_cvt_in_batch(int prec, void* const* dst, const double* const* src, const size_t* count, const size_t* lo_off,
-                                int nseg, cudaStream_t stream, int background_ctas)
+template <typename SRC>
+static void launch_in_batch(int prec, const CastBatch& cb, int grid, cudaStream_t stream)
+{
+    if (prec == SDPA_PREC_BF16X3) cvt_in_batch_kernel<SRC, 2><<<grid, kCastThreads, 0, stream>>>(cb);
+    else if (prec == SDPA_PREC_BF16) cvt_in_batch_kernel<SRC, 1><<<grid, kCastThreads, 0, stream>>>(cb);
+    else cvt_in_batch_kernel<SRC, 0><<<grid, kCastThreads, 0, stream>>>(cb);
+}
+template <typename SRC>
+static void launch_typed_scalar(int prec, void* dst, size_t lo_off, const void* src, size_t count, cudaStream_t stream)
+{
+    const SRC* s = reinterpret_cast<const SRC*>(src);
+    if (prec == SDPA_PREC_BF16X3) cvt_typed_scalar_kernel<SRC, 2><<<cast_grid(count), kCastThreads, 0, stream>>>(dst, lo_off, s, count);
+    else if (prec == SDPA_PREC_BF16) cvt_typed_scalar_kernel<SRC, 1><<<cast_grid(count), kCastThreads, 0, stream>>>(dst, lo_off, s, count);
+    else cvt_typed_scalar_kernel<SRC, 0><<<cast_grid(count), kCastThreads, 0, stream>>>(dst, lo_off, s, count);
+}
+
+// Up to three operands in one launch; falls back to one launch per operand when a pointer is not aligned to a 2-element unit
+// (16 B for fp64 sources) or a count is odd (the batched kernel moves 2-element units only).
+sdpa_status launch_cvt_in_batch(int src_dtype, int prec, void* const* dst, const void* const* src, const size_t* count,
+                                const size_t* lo_off, int nseg, cudaStream_t stream, int background_ctas)
 {
     if (nseg < 0 || nseg > 3) {
         set_error("launch_cvt_in_batch: 0..3 segments");
         return SDPA_ERR_INVALID;
     }
+    if (src_dtype != SDPA_DTYPE_F64 && src_dtype != SDPA_DTYPE_F32 && src_dtype != SDPA_DTYPE_BF16) {
+        set_error("launch_cvt_in_batch: unknown source dtype %d", src_dtype);
+        return SDPA_ERR_INVALID;
+    }
+    if (src_dtype != SDPA_DTYPE_F64 && background_ctas > 0) {   // typed passes never cast ahead
+        set_error("launch_cvt_in_batch: the background form takes fp64 sources only");
+        return SDPA_ERR_INVALID;
+    }
+    const size_t src_unit = src_dtype == SDPA_DTYPE_F64 ? 16 : (src_dtype == SDPA_DTYPE_F32 ? 8 : 4);
     bool vec_ok = true;
     size_t units_total = 0;
     CastBatch cb;
@@ -493,7 +575,7 @@ sdpa_status launch_cvt_in_batch(int prec, void* const* dst, const double* const*
     const bool split = prec == SDPA_PREC_BF16X3;
     for (int k = 0; k < nseg; ++k) {
         if (count[k] == 0) continue;
-        vec_ok = vec_ok && (count[k] % 2 == 0) && aligned(src[k], 16) && aligned(dst[k], 8) && (!split || (lo_off && lo_off[k] % 2 == 0));
+        vec_ok = vec_ok && (count[k] % 2 == 0) && aligned(src[k], src_unit) && aligned(dst[k], 8) && (!split || (lo_off && lo_off[k] % 2 == 0));
         cb.dst[k] = dst[k];
         cb.src[k] = src[k];
         cb.units[k] = count[k] / 2;
@@ -503,11 +585,21 @@ sdpa_status launch_cvt_in_batch(int prec, void* const* dst, const double* const*
     if (units_total == 0 && vec_ok) return SDPA_OK;
     if (!vec_ok) {
         for (int k = 0; k < nseg; ++k) {
+            if (src_dtype != SDPA_DTYPE_F64) {
+                if (count[k] == 0) continue;
+                const size_t lo = split && lo_off ? lo_off[k] : 0;
+                if (src_dtype == SDPA_DTYPE_F32) launch_typed_scalar<float>(prec, dst[k], lo, src[k], count[k], stream);
+                else launch_typed_scalar<__nv_bfloat16>(prec, dst[k], lo, src[k], count[k], stream);
+                count_launch();
+                SDPA_CUDA_TRY(cudaGetLastError());
+                continue;
+            }
+            const double* s = reinterpret_cast<const double*>(src[k]);
             if (split) {
                 __nv_bfloat16* hi = reinterpret_cast<__nv_bfloat16*>(dst[k]);
-                SDPA_TRY(launch_cvt_d2bf16x2(hi, hi + (lo_off ? lo_off[k] : 0), src[k], count[k], stream));
-            } else if (prec == SDPA_PREC_BF16) SDPA_TRY(launch_cvt_d2bf16(reinterpret_cast<__nv_bfloat16*>(dst[k]), src[k], count[k], stream));
-            else SDPA_TRY(launch_cvt_d2f(reinterpret_cast<float*>(dst[k]), src[k], count[k], stream));
+                SDPA_TRY(launch_cvt_d2bf16x2(hi, hi + (lo_off ? lo_off[k] : 0), s, count[k], stream));
+            } else if (prec == SDPA_PREC_BF16) SDPA_TRY(launch_cvt_d2bf16(reinterpret_cast<__nv_bfloat16*>(dst[k]), s, count[k], stream));
+            else SDPA_TRY(launch_cvt_d2f(reinterpret_cast<float*>(dst[k]), s, count[k], stream));
         }
         return SDPA_OK;
     }
@@ -536,9 +628,9 @@ sdpa_status launch_cvt_in_batch(int prec, void* const* dst, const double* const*
         return SDPA_OK;
     }
     const int grid = cast_grid(units_total / kUnroll);
-    if (split) cvt_in_batch_kernel<2><<<grid, kCastThreads, 0, stream>>>(cb);
-    else if (prec == SDPA_PREC_BF16) cvt_in_batch_kernel<1><<<grid, kCastThreads, 0, stream>>>(cb);
-    else cvt_in_batch_kernel<0><<<grid, kCastThreads, 0, stream>>>(cb);
+    if (src_dtype == SDPA_DTYPE_F64) launch_in_batch<double>(prec, cb, grid, stream);
+    else if (src_dtype == SDPA_DTYPE_F32) launch_in_batch<float>(prec, cb, grid, stream);
+    else launch_in_batch<__nv_bfloat16>(prec, cb, grid, stream);
     count_launch();
     SDPA_CUDA_TRY(cudaGetLastError());
     return SDPA_OK;

@@ -61,7 +61,7 @@ sdpa_status launch_cvt_d2bf16(__nv_bfloat16* dst, const double* src, size_t coun
 sdpa_status launch_cvt_d2bf16x2(__nv_bfloat16* dst_hi, __nv_bfloat16* dst_lo, const double* src, size_t count, cudaStream_t stream);
 struct CastBatch {
     void* dst[3];
-    const double* src[3];
+    const void* src[3];   // element type: the launch's source dtype
     size_t units[3];   // 2-element units per segment
     size_t lo_off[3];  // split precision: distance from the hi to the lo array, in 2-element units
     unsigned long long* trace;   // developer aid (background form): per CTA [start, end] %globaltimer stamps, or NULL
@@ -70,11 +70,12 @@ struct CastBatch {
 // stamps %globaltimer into *dst in stream order.
 void set_cast_trace(unsigned long long* buf);
 sdpa_status launch_stamp(unsigned long long* dst, cudaStream_t stream);
+// src_dtype: sdpa_dtype of the sources (fp64, fp32 or bf16); prec: the compute precision written.
 // lo_off (elements, per segment) is read for SDPA_PREC_BF16X3 only and may be NULL otherwise.
-sdpa_status launch_cvt_in_batch(int prec, void* const* dst, const double* const* src, const size_t* count, const size_t* lo_off,
-                                int nseg, cudaStream_t stream, int background_ctas = 0);
-// background_ctas > 0: the small-footprint form (that many CTAs of 128 threads, 40 KB of shared memory, <= 32 registers) that
-// fits on an SM beside a resident CTA of the persistent fused kernel.
+sdpa_status launch_cvt_in_batch(int src_dtype, int prec, void* const* dst, const void* const* src, const size_t* count,
+                                const size_t* lo_off, int nseg, cudaStream_t stream, int background_ctas = 0);
+// background_ctas > 0 (fp64 sources only): the small-footprint form (that many CTAs of 128 threads, 40 KB of shared memory,
+// <= 32 registers) that fits on an SM beside a resident CTA of the persistent fused kernel.
 
 // fp32 CUDA-core fused attention.  Q [rows x dk], K [n x dk], V [n x dv] fp32 row-major.
 // If out64 != nullptr (requires splits == 1) the normalised result is written as fp64

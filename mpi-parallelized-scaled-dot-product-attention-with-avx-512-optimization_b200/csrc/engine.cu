@@ -197,9 +197,13 @@ struct Shard {
     DevBuf out32[2], out64[2];                  // root: reduced fp32 batch / fp64 batch for D2H
     cudaEvent_t ev_compute_done[2] = {nullptr, nullptr}, ev_slot_free[2] = {nullptr, nullptr};
     cudaEvent_t ev_comm_done[2] = {nullptr, nullptr};
+    // what the fused kernel reads as K / V: the resident Kc / Vc, or the caller's arrays when they already are in compute
+    // precision (typed passes: bf16 operands at BF16, fp32 operands at F32 -- no cast at all)
+    const void* k_in = nullptr;
+    const void* v_in = nullptr;
     // K/V casts of a device-resident call that wait for the first Q batch so that all three share one launch
     void* pend_dst[2] = {nullptr, nullptr};
-    const double* pend_src[2] = {nullptr, nullptr};
+    const void* pend_src[2] = {nullptr, nullptr};   // element type: sdpa_ctx::dtype
     size_t pend_cnt[2] = {0, 0};
     int npend = 0;
     cudaEvent_t ev_join[3] = {nullptr, nullptr, nullptr};
@@ -239,6 +243,8 @@ struct sdpa_ctx {
     int rank_base = 0;
     int dk = 0, dv = 0;
     int prec = SDPA_PREC_F32;   // resolved precision of the resident shard
+    int dtype = SDPA_DTYPE_F64; // element type of the operands and the result of the pass the shard was loaded for
+    bool zero_copy = false;     // the fused kernel reads the caller's K/V/Q in place (Shard::k_in / v_in, Q per batch)
     int q_batch = 0;
     bool peer_ok = false;
     float last_timing[6] = {0, 0, 0, 0, 0, 0};
@@ -250,10 +256,11 @@ struct sdpa_ctx {
     // several processes sdpa_synchronize is collective like the passes themselves).  SDPA_DEFER_TWIN=0 keeps the twin in the stream.
     struct GuardRef { int shard; unsigned int slot, epoch; };
     struct PendingPass {
-        std::vector<const double*> K, V, Q;   // per local shard
+        int dtype;                           // re-run as the same typed pass
+        std::vector<const void*> K, V, Q;     // per local shard
         std::vector<int> n_local;
         int dk, dv;
-        double* result; int m;
+        void* result; int m;
         std::vector<GuardRef> guards;         // every fused launch of the pass
     };
     std::vector<PendingPass> pending;
@@ -426,12 +433,22 @@ static sdpa_status cast_in(int prec, void* dst, size_t lo_off, size_t at, const 
 }
 
 // AUTO keeps the reference's accuracy class (fp32, attention-mpi.c:168-189): the split-precision tensor-core kernel where
-// the shape allows it, else the fp32 CUDA-core kernel.  Plain bf16 is opt-in only: its operand rounding can move peaky
-// scores beyond the reference's own 0.02 acceptance gate (attention-mpi.c:476).
-static int resolve_precision(int requested, int dk, int dv)
+// the shape allows it, else the fp32 CUDA-core kernel.  Plain bf16 is opt-in only for fp64 and fp32 operands: its operand
+// rounding can move peaky scores beyond the reference's own 0.02 acceptance gate (attention-mpi.c:476).  bf16 operands have
+// been rounded by the caller already, so for them AUTO is the bf16 kernel, which reads them in place.
+static int resolve_precision(int dtype, int requested, int dk, int dv)
 {
     if (requested == SDPA_PREC_BF16 || requested == SDPA_PREC_F32 || requested == SDPA_PREC_BF16X3) return requested;
+    if (dtype == SDPA_DTYPE_BF16) return attn_umma_supported(dk, dv, 1) ? SDPA_PREC_BF16 : SDPA_PREC_F32;
     return attn_umma_supported(dk, dv, 2) ? SDPA_PREC_BF16X3 : SDPA_PREC_F32;
+}
+static bool dtype_valid(int dtype) { return dtype == SDPA_DTYPE_F64 || dtype == SDPA_DTYPE_F32 || dtype == SDPA_DTYPE_BF16; }
+static size_t dtype_size(int dtype) { return dtype == SDPA_DTYPE_F64 ? 8 : (dtype == SDPA_DTYPE_F32 ? 4 : 2); }
+static const char* dtype_name(int dtype) { return dtype == SDPA_DTYPE_F64 ? "fp64" : (dtype == SDPA_DTYPE_F32 ? "fp32" : "bf16"); }
+// Operands that already are in compute precision: the fused kernel reads the caller's arrays, no cast kernel runs.
+static bool reads_in_place(int dtype, int prec)
+{
+    return (dtype == SDPA_DTYPE_BF16 && prec == SDPA_PREC_BF16) || (dtype == SDPA_DTYPE_F32 && prec == SDPA_PREC_F32);
 }
 static sdpa_status check_precision(int prec, int dk, int dv)
 {
@@ -537,18 +554,22 @@ static sdpa_status upload_cast(Shard& s, int prec, void* dst, size_t lo_off, con
     return SDPA_OK;
 }
 
-static sdpa_status load_kv(sdpa_ctx* ctx, const double* const* K_shards, const double* const* V_shards,
+static sdpa_status load_kv(sdpa_ctx* ctx, int dtype, const void* const* K_shards, const void* const* V_shards,
                            const int* n_local, int dk, int dv, bool on_device, bool defer_casts = false, bool ahead = false)
 {
     if (!ctx || !n_local || dk < 1 || dv < 1) {
         set_error("load_kv: bad arguments");
         return SDPA_ERR_INVALID;
     }
-    const int prec = resolve_precision(ctx->cfg.precision, dk, dv);
+    const int prec = resolve_precision(dtype, ctx->cfg.precision, dk, dv);
     SDPA_TRY(check_precision(prec, dk, dv));
+    // typed passes (device arrays, deferred casts) whose operands already are in compute precision: no resident copy
+    const bool zero_copy = on_device && defer_casts && reads_in_place(dtype, prec);
     ctx->dk = dk;
     ctx->dv = dv;
     ctx->prec = prec;
+    ctx->dtype = dtype;
+    ctx->zero_copy = zero_copy;
     ctx->qshard = false;   // sdpa_load_kv_host_full sets it again when it replicates
     const size_t esz = elem_size(prec);
     for (size_t i = 0; i < ctx->shards.size(); ++i) {
@@ -565,25 +586,35 @@ static sdpa_status load_kv(sdpa_ctx* ctx, const double* const* K_shards, const d
             std::swap(s.Vc, s.VcAlt);
             s.kv_set ^= 1;
         }
-        // +128 rows of slack so TMA boxes / vector loads past the last row stay in bounds
-        SDPA_TRY(s.Kc.reserve(((size_t)s.n_local + 128) * dk * esz));
-        SDPA_TRY(s.Vc.reserve(((size_t)s.n_local + 128) * dv * esz));
-        s.k_lo_off = ((size_t)s.n_local + 128) * dk;
-        s.v_lo_off = ((size_t)s.n_local + 128) * dv;
         s.npend = 0;
-        if (s.n_local > 0 && on_device && defer_casts) {
-            // sdpa_attention_device_full: the sources stay valid for the whole call, so the casts ride with Q's
+        if (zero_copy && s.n_local > 0) {
+            // the kernels read the caller's rows; TMA zero-fills the boxes past row n_local, the fp32 kernel masks them
+            s.k_in = K_shards[i];
+            s.v_in = V_shards[i];
+        } else {
+            // +128 rows of slack so TMA boxes / vector loads past the last row stay in bounds
+            SDPA_TRY(s.Kc.reserve(((size_t)s.n_local + 128) * dk * esz));
+            SDPA_TRY(s.Vc.reserve(((size_t)s.n_local + 128) * dv * esz));
+            s.k_lo_off = ((size_t)s.n_local + 128) * dk;
+            s.v_lo_off = ((size_t)s.n_local + 128) * dv;
+            s.k_in = s.Kc.p;
+            s.v_in = s.Vc.p;
+        }
+        if (zero_copy || s.n_local == 0) {
+            // nothing to cast
+        } else if (on_device && defer_casts) {
+            // sdpa_attention_device_full / _typed: the sources stay valid for the whole call, so the casts ride with Q's
             s.pend_dst[0] = s.Kc.p, s.pend_src[0] = K_shards[i], s.pend_cnt[0] = (size_t)s.n_local * dk;
             s.pend_dst[1] = s.Vc.p, s.pend_src[1] = V_shards[i], s.pend_cnt[1] = (size_t)s.n_local * dv;
             s.npend = 2;
-        } else if (s.n_local > 0) {
-            SDPA_TRY(upload_cast(s, prec, s.Kc.p, s.k_lo_off, K_shards[i], (size_t)s.n_local * dk, on_device));
-            SDPA_TRY(upload_cast(s, prec, s.Vc.p, s.v_lo_off, V_shards[i], (size_t)s.n_local * dv, on_device));
+        } else {   // fp64 only: sdpa_load_kv_host / sdpa_load_kv_device
+            SDPA_TRY(upload_cast(s, prec, s.Kc.p, s.k_lo_off, static_cast<const double*>(K_shards[i]), (size_t)s.n_local * dk, on_device));
+            SDPA_TRY(upload_cast(s, prec, s.Vc.p, s.v_lo_off, static_cast<const double*>(V_shards[i]), (size_t)s.n_local * dv, on_device));
         }
         if (is_umma(prec)) {
             if (!s.plan) SDPA_TRY(umma_plan_create(&s.plan));
-            SDPA_TRY(umma_plan_bind_kv(s.plan, s.Kc.as<__nv_bfloat16>(), s.Vc.as<__nv_bfloat16>(), s.n_local, dk, dv, prec_hl(prec),
-                                       s.k_lo_off, s.v_lo_off));
+            SDPA_TRY(umma_plan_bind_kv(s.plan, static_cast<const __nv_bfloat16*>(s.k_in), static_cast<const __nv_bfloat16*>(s.v_in),
+                                       s.n_local, dk, dv, prec_hl(prec), s.k_lo_off, s.v_lo_off));
         }
     }
     // Host sources: block until the uploads have been consumed (the caller may reuse its arrays).
@@ -663,13 +694,14 @@ static sdpa_status reserve_batch_buffers(sdpa_ctx* ctx, Shard& s, int B, int spl
     return SDPA_OK;
 }
 
-// The fused kernel for one batch on one shard: fills the split partials, or writes fp64 directly.
-static sdpa_status run_fused(sdpa_ctx* ctx, Shard& s, int slot, int rows, int splits, Partials part, double* direct_out)
+// The fused kernel for one batch on one shard: fills the split partials, or writes fp64 directly.  q_f32: the fp32 Q rows of
+// the batch (the fp32 kernel; the tensor-core kernels read Q through the plan's map of the slot).
+static sdpa_status run_fused(sdpa_ctx* ctx, Shard& s, int slot, const float* q_f32, int rows, int splits, Partials part, double* direct_out)
 {
     if (is_umma(ctx->prec)) {
         return launch_attn_umma(s.plan, slot, rows, splits, part, direct_out, s.sm_count, s.s_compute);
     }
-    return launch_attn_f32(s.qc[slot].as<float>(), s.Kc.as<float>(), s.Vc.as<float>(), rows, s.n_local, ctx->dk,
+    return launch_attn_f32(q_f32, static_cast<const float*>(s.k_in), static_cast<const float*>(s.v_in), rows, s.n_local, ctx->dk,
                            ctx->dv, splits, part, direct_out, s.s_compute);
 }
 
@@ -831,9 +863,11 @@ static sdpa_status ipc_setup(sdpa_ctx* ctx, int rows_cap, int dv)
     return SDPA_OK;
 }
 
-static sdpa_status attention_impl(sdpa_ctx* ctx, const double* Q_host, const double* const* Q_dev,
-                                  double* result, bool result_on_device, int m, bool q_from_root = false,
-                                  bool blocking = true)
+// Q_dev / result: element type `dtype` (device arrays; host arrays are fp64).  A typed result is merged into the root's fp64
+// batch slot and rounded from there into the caller's array.
+static sdpa_status attention_impl(sdpa_ctx* ctx, const double* Q_host, const void* const* Q_dev,
+                                  void* result, bool result_on_device, int m, bool q_from_root = false,
+                                  bool blocking = true, int dtype = SDPA_DTYPE_F64)
 {
     if (!ctx || m < 0) {
         set_error("attention: bad arguments");
@@ -841,6 +875,10 @@ static sdpa_status attention_impl(sdpa_ctx* ctx, const double* Q_host, const dou
     }
     if (ctx->dk == 0) {
         set_error("attention: no K/V shard loaded (call sdpa_load_kv_* first)");
+        return SDPA_ERR_INVALID;
+    }
+    if (dtype != ctx->dtype) {
+        set_error("attention: the K/V shard was loaded for %s operands, this call passes %s arrays", dtype_name(ctx->dtype), dtype_name(dtype));
         return SDPA_ERR_INVALID;
     }
     const bool on_device = Q_dev != nullptr;
@@ -872,7 +910,7 @@ static sdpa_status attention_impl(sdpa_ctx* ctx, const double* Q_host, const dou
             if (s.npend == 0) continue;
             SDPA_CUDA_TRY(cudaSetDevice(s.dev));
             const size_t lo[2] = {s.k_lo_off, s.v_lo_off};
-            SDPA_TRY(launch_cvt_in_batch(ctx->prec, s.pend_dst, s.pend_src, s.pend_cnt, lo, 2, s.s_compute));
+            SDPA_TRY(launch_cvt_in_batch(ctx->dtype, ctx->prec, s.pend_dst, s.pend_src, s.pend_cnt, lo, 2, s.s_compute));
             s.npend = 0;
             s.ahead_call = false;
             s.kv_guard[s.kv_set] = nullptr;
@@ -929,6 +967,10 @@ static sdpa_status attention_impl(sdpa_ctx* ctx, const double* Q_host, const dou
     const bool use_in = !on_device;                                  // H2D of the Q batches
     const bool use_comm = world > 1;                                 // collectives / peer merge
     const bool use_out = world > 1 || !result_on_device;             // D2H of the result, slot recycling
+    // where the merged fp64 rows go: straight into an fp64 device result, else the root's batch slot out64[b] (then D2H, or
+    // rounded into the typed result)
+    const bool direct = result_on_device && dtype == SDPA_DTYPE_F64;
+    double* const res64 = static_cast<double*>(result);
     for (int i = 0; i < L; ++i) {
         Shard& s = ctx->shards[i];
         SDPA_CUDA_TRY(cudaSetDevice(s.dev));
@@ -943,7 +985,7 @@ static sdpa_status attention_impl(sdpa_ctx* ctx, const double* Q_host, const dou
         if (!(s.last_call_queued && !blocking && s.marks_on && marked)) compute_stream_touched(s);
         s.marks_on = marked;
         s.q_lo_off = (size_t)(((B + 127) & ~127) + 128) * dk;
-        if (is_umma(ctx->prec))
+        if (is_umma(ctx->prec) && dtype == SDPA_DTYPE_F64)   // typed passes bind their Q rows batch by batch (below)
             for (int b = 0; b < 2; ++b)
                 SDPA_TRY(umma_plan_bind_q(s.plan, b, s.qc[b].as<__nv_bfloat16>(), (B + 127) & ~127, dk, prec_hl(ctx->prec), s.q_lo_off));
         SDPA_TRY(time_begin(s, 3, s.s_compute));
@@ -987,10 +1029,10 @@ static sdpa_status attention_impl(sdpa_ctx* ctx, const double* Q_host, const dou
             Shard& s = ctx->shards[i];
             SDPA_CUDA_TRY(cudaSetDevice(s.dev));
             const bool single = (world == 1);
-            const double* q_src_dev = nullptr;
+            const void* q_src_dev = nullptr;   // element type `dtype`
             const bool have_q = !q_from_root || s.grank == 0;  // q_from_root: only shard 0's process holds Q
             if (on_device) {
-                q_src_dev = Q_dev[i] + (size_t)row0 * dk;
+                q_src_dev = static_cast<const char*>(Q_dev[i]) + (size_t)row0 * dk * dtype_size(dtype);
             } else if (have_q) {
                 // copy stream: wait until the cast of batch ii-2 released this buffer
                 if (ii >= 2) SDPA_CUDA_TRY(cudaStreamWaitEvent(s.s_in, s.ev_q_free[b], 0));
@@ -1017,17 +1059,30 @@ static sdpa_status attention_impl(sdpa_ctx* ctx, const double* Q_host, const dou
                 if (s.plain_end_recorded) SDPA_CUDA_TRY(cudaStreamWaitEvent(s.s_cast, s.ev_plain_end, 0));
                 s.ahead_ever = true;
             }
-            SDPA_TRY(time_begin(s, 0, cst));
-            if (s.npend > 0) {
+            // Typed passes: the tensor-core kernels get a map of exactly this batch's Q rows -- the caller's (zero copy: no cast
+            // stage at all) or the slot's -- so the rows of a 256-row block past the batch are zero-filled by TMA and never
+            // stale slot contents (which the overflow guard would look at too).  Zero copy on the fp32 kernel: Q read in place.
+            if (dtype != SDPA_DTYPE_F64 && is_umma(ctx->prec))
+                SDPA_TRY(umma_plan_bind_q(s.plan, b, ctx->zero_copy ? static_cast<const __nv_bfloat16*>(q_src_dev) : s.qc[b].as<__nv_bfloat16>(),
+                                          bs, dk, prec_hl(ctx->prec), s.q_lo_off));
+            if (!ctx->zero_copy) SDPA_TRY(time_begin(s, 0, cst));
+            if (ctx->zero_copy) {
+                // nothing to cast
+            } else if (s.npend > 0) {
                 void* cd[3] = {s.pend_dst[0], s.pend_dst[1], s.qc[b].p};
-                const double* cs[3] = {s.pend_src[0], s.pend_src[1], q_src_dev};
+                const void* cs[3] = {s.pend_src[0], s.pend_src[1], q_src_dev};
                 const size_t cc[3] = {s.pend_cnt[0], s.pend_cnt[1], (size_t)bs * dk};
                 const size_t lo[3] = {s.k_lo_off, s.v_lo_off, s.q_lo_off};
-                SDPA_TRY(launch_cvt_in_batch(ctx->prec, cd, cs, cc, lo, have_q ? 3 : 2, cst, cast_aside ? s.sm_count : 0));
+                SDPA_TRY(launch_cvt_in_batch(dtype, ctx->prec, cd, cs, cc, lo, have_q ? 3 : 2, cst, cast_aside ? s.sm_count : 0));
                 s.npend = 0;
                 ++all_launches;
+            } else if (have_q && dtype != SDPA_DTYPE_F64) {
+                void* cd[1] = {s.qc[b].p};
+                const size_t cc[1] = {(size_t)bs * dk}, lo[1] = {s.q_lo_off};
+                SDPA_TRY(launch_cvt_in_batch(dtype, ctx->prec, cd, &q_src_dev, cc, lo, 1, s.s_compute));
+                ++all_launches;
             } else if (have_q) {
-                SDPA_TRY(cast_in(ctx->prec, s.qc[b].p, s.q_lo_off, 0, q_src_dev, (size_t)bs * dk, s.s_compute));
+                SDPA_TRY(cast_in(ctx->prec, s.qc[b].p, s.q_lo_off, 0, static_cast<const double*>(q_src_dev), (size_t)bs * dk, s.s_compute));
                 ++all_launches;
             }
             if (q_from_root) {  // the Q batch travels in compute precision (mpi.c:305,327: Ibcast of the fp32 batch)
@@ -1038,7 +1093,7 @@ static sdpa_status attention_impl(sdpa_ctx* ctx, const double* Q_host, const dou
                     SDPA_NCCL_TRY(api->Broadcast(lo, lo, (size_t)bs * dk * 2, ncclUint8, 0, s.comm, s.s_compute));
                 }
             }
-            SDPA_TRY(time_end(s, 0, cst));
+            if (!ctx->zero_copy) SDPA_TRY(time_end(s, 0, cst));
             if (cast_aside) {
                 SDPA_CUDA_TRY(cudaEventRecord(s.ev_cast_done, s.s_cast));
                 SDPA_CUDA_TRY(cudaStreamWaitEvent(s.s_compute, s.ev_cast_done, 0));
@@ -1048,11 +1103,12 @@ static sdpa_status attention_impl(sdpa_ctx* ctx, const double* Q_host, const dou
 
             Partials part{s.part_o.as<float>(), s.part_tmax.as<float>(), s.part_lsum.as<float>(), splits, B};
             double* final_dst = nullptr;  // where the fp64 rows of this batch go when no cross-GPU merge is needed
-            if (single) final_dst = result_on_device ? result + (size_t)row0 * dv : s.out64[b].as<double>();
+            if (single) final_dst = direct ? res64 + (size_t)row0 * dv : s.out64[b].as<double>();
 
             SDPA_TRY(time_begin(s, 1, s.s_compute));
             if (ctx->cast_trace.p) SDPA_TRY(launch_stamp(ctx->cast_trace.as<unsigned long long>() + 600 + 2 * (ctx->trace_pass & 1), s.s_compute));
-            SDPA_TRY(run_fused(ctx, s, b, bs, splits, part, (single && splits == 1) ? final_dst : nullptr));
+            const float* q_f32 = ctx->zero_copy ? static_cast<const float*>(q_src_dev) : s.qc[b].as<float>();
+            SDPA_TRY(run_fused(ctx, s, b, q_f32, bs, splits, part, (single && splits == 1) ? final_dst : nullptr));
             if (ctx->cast_trace.p) SDPA_TRY(launch_stamp(ctx->cast_trace.as<unsigned long long>() + 601 + 2 * (ctx->trace_pass++ & 1), s.s_compute));
             SDPA_TRY(time_end(s, 1, s.s_compute));
             ++fused_launches;
@@ -1127,7 +1183,7 @@ static sdpa_status attention_impl(sdpa_ctx* ctx, const double* Q_host, const dou
                             sync.block_counter = x.flags.as<unsigned int>() + 4 + b;
                             sync.epoch = x.epoch;
                             sync.trace = x.trace_slot(x.epoch);
-                            double* dst = result_on_device ? result + (size_t)row0 * dv : s.out64[b].as<double>();
+                            double* dst = direct ? res64 + (size_t)row0 * dv : s.out64[b].as<double>();
                             SDPA_TRY(launch_merge_root_instream(part, pieces ? &wm : nullptr, max_pieces, guard, guard_epoch, cp, tp, lp, world - 1, bs,
                                                                 dv, dst, sync, s.s_compute));
                         } else if (x.push) {
@@ -1226,7 +1282,7 @@ static sdpa_status attention_impl(sdpa_ctx* ctx, const double* Q_host, const dou
                     col.consumed = x.flags.as<unsigned int>() + 2 + b;
                     col.block_counter = x.flags.as<unsigned int>() + 8 + b;
                     col.epoch = x.epoch;
-                    double* dst = result_on_device ? result + (size_t)row0 * dv : s.out64[b].as<double>();
+                    double* dst = direct ? res64 + (size_t)row0 * dv : s.out64[b].as<double>();
                     SDPA_TRY(launch_collect_slices(dst, x.stage[b].as<double>(), bs, dv, col, world, s.s_comm));
                 }
                 SDPA_TRY(time_end(s, 2, s.s_comm));
@@ -1251,7 +1307,7 @@ static sdpa_status attention_impl(sdpa_ctx* ctx, const double* Q_host, const dou
                 sync.block_counter = x.flags.as<unsigned int>() + 4 + b;
                 sync.epoch = x.epoch;
                 sync.trace = x.trace_slot(x.epoch);
-                double* dst = result_on_device ? result + (size_t)row0 * dv : s.out64[b].as<double>();
+                double* dst = direct ? res64 + (size_t)row0 * dv : s.out64[b].as<double>();
                 SDPA_TRY(time_begin(s, 2, s.s_compute));
                 SDPA_TRY(launch_merge_peers_synced(cp, tp, lp, world, bs, dv, dst, sync, s.s_compute));
                 SDPA_TRY(time_end(s, 2, s.s_compute));
@@ -1269,7 +1325,7 @@ static sdpa_status attention_impl(sdpa_ctx* ctx, const double* Q_host, const dou
                 SDPA_CUDA_TRY(cudaStreamWaitEvent(s.s_comm, s.ev_compute_done[b], 0));
                 unsigned int* consumed[64];
                 for (int r = 0; r < world; ++r) consumed[r] = x.peer_flags[r] + 2 + b;
-                double* dst = result_on_device ? result + (size_t)row0 * dv : s.out64[b].as<double>();
+                double* dst = direct ? res64 + (size_t)row0 * dv : s.out64[b].as<double>();
                 SDPA_TRY(time_begin(s, 2, s.s_comm));
                 SDPA_TRY(launch_merge_inbox_background(x.xbuf[b].as<float>(), (size_t)x.cap_rows * ((size_t)dv + 2), x.cap_rows, world,
                                                        x.flags.as<unsigned int>() + sdpa_ctx::Ipc::kFlagReady + b * 64, consumed,
@@ -1297,7 +1353,7 @@ static sdpa_status attention_impl(sdpa_ctx* ctx, const double* Q_host, const dou
                 sync.block_counter = x.flags.as<unsigned int>() + 4 + b;
                 sync.epoch = x.epoch;
                 sync.trace = x.trace_slot(x.epoch);
-                double* dst = result_on_device ? result + (size_t)row0 * dv : s.out64[b].as<double>();
+                double* dst = direct ? res64 + (size_t)row0 * dv : s.out64[b].as<double>();
                 SDPA_TRY(time_begin(s, 2, s.s_comm));
                 SDPA_TRY(launch_merge_peers_synced(cp, tp, lp, world, bs, dv, dst, sync, s.s_comm));
                 SDPA_TRY(time_end(s, 2, s.s_comm));
@@ -1320,7 +1376,7 @@ static sdpa_status attention_impl(sdpa_ctx* ctx, const double* Q_host, const dou
                 tp[i] = ctx->shards[i].tmax[b].as<float>();
                 lp[i] = ctx->shards[i].lsum[b].as<float>();
             }
-            double* dst = result_on_device ? result + (size_t)row0 * dv : r.out64[b].as<double>();
+            double* dst = direct ? res64 + (size_t)row0 * dv : r.out64[b].as<double>();
             SDPA_TRY(time_begin(r, 2, r.s_comm));
             SDPA_TRY(launch_merge_peers(cp, tp, lp, L, bs, dv, dst, r.s_comm));
             SDPA_TRY(time_end(r, 2, r.s_comm));
@@ -1369,7 +1425,7 @@ static sdpa_status attention_impl(sdpa_ctx* ctx, const double* Q_host, const dou
                     Shard& s = ctx->shards[i];
                     SDPA_CUDA_TRY(cudaSetDevice(s.dev));
                     if (s.grank == 0) {
-                        double* dst = result_on_device ? result + (size_t)row0 * dv : s.out64[b].as<double>();
+                        double* dst = direct ? res64 + (size_t)row0 * dv : s.out64[b].as<double>();
                         SDPA_TRY(launch_finalize_reduced(dst, s.out32[b].as<float>(), s.out32[b].as<float>() + (size_t)bs * dv, bs, dv, s.s_comm));
                     }
                     SDPA_TRY(time_end(s, 2, s.s_comm));
@@ -1406,7 +1462,7 @@ static sdpa_status attention_impl(sdpa_ctx* ctx, const double* Q_host, const dou
                 Shard& s = ctx->shards[i];
                 SDPA_CUDA_TRY(cudaSetDevice(s.dev));
                 if (s.grank == 0) {
-                    double* dst = result_on_device ? result + (size_t)row0 * dv : s.out64[b].as<double>();
+                    double* dst = direct ? res64 + (size_t)row0 * dv : s.out64[b].as<double>();
                     SDPA_TRY(launch_cvt_f2d(dst, s.out32[b].as<float>(), (size_t)bs * dv, s.s_comm));  // mpi.c:373
                 }
                 SDPA_TRY(time_end(s, 2, s.s_comm));
@@ -1416,17 +1472,24 @@ static sdpa_status attention_impl(sdpa_ctx* ctx, const double* Q_host, const dou
             }
         }
 
-        // ---- root: fp64 rows of this batch back to the host ------------------------------------
+        // ---- root: fp64 rows of this batch back to the host, or rounded into the typed result ------------
         for (int i = 0; i < L; ++i) {
             Shard& s = ctx->shards[i];
-            if (s.grank != 0 || !use_out) continue;   // single GPU writing to device memory: all on the compute stream
+            if (s.grank != 0) continue;
+            // one GPU writing to device memory: all on the compute stream (fp64 rows are in place already)
+            cudaStream_t st = use_out ? s.s_out : s.s_compute;
+            if (!use_out && direct) continue;
             SDPA_CUDA_TRY(cudaSetDevice(s.dev));
-            cudaEvent_t ready = world > 1 ? s.ev_comm_done[b] : s.ev_compute_done[b];
-            SDPA_CUDA_TRY(cudaStreamWaitEvent(s.s_out, ready, 0));
+            if (use_out) SDPA_CUDA_TRY(cudaStreamWaitEvent(s.s_out, world > 1 ? s.ev_comm_done[b] : s.ev_compute_done[b], 0));
             if (!result_on_device)
-                SDPA_CUDA_TRY(cudaMemcpyAsync(result + (size_t)row0 * dv, s.out64[b].p, (size_t)bs * dv * sizeof(double),
+                SDPA_CUDA_TRY(cudaMemcpyAsync(res64 + (size_t)row0 * dv, s.out64[b].p, (size_t)bs * dv * sizeof(double),
                                               cudaMemcpyDeviceToHost, s.s_out));
-            SDPA_CUDA_TRY(cudaEventRecord(s.ev_slot_free[b], s.s_out));
+            else if (dtype == SDPA_DTYPE_F32)
+                SDPA_TRY(launch_cvt_d2f(static_cast<float*>(result) + (size_t)row0 * dv, s.out64[b].as<double>(), (size_t)bs * dv, st));
+            else if (dtype == SDPA_DTYPE_BF16)
+                SDPA_TRY(launch_cvt_d2bf16(static_cast<__nv_bfloat16*>(result) + (size_t)row0 * dv, s.out64[b].as<double>(), (size_t)bs * dv, st));
+            if (use_out) SDPA_CUDA_TRY(cudaEventRecord(s.ev_slot_free[b], s.s_out));
+            else compute_stream_touched(s);
         }
         if (seq_slots) ++ctx->batch_seq;
     }
@@ -1569,7 +1632,7 @@ static sdpa_status attention_qshard_host(sdpa_ctx* ctx, const double* Q, double*
             Partials part{s.part_o.as<float>(), s.part_tmax.as<float>(), s.part_lsum.as<float>(), splits, B};
             double* dst = s.out64[b].as<double>();
             SDPA_TRY(time_begin(s, 1, s.s_compute));
-            SDPA_TRY(run_fused(ctx, s, b, bs, splits, part, splits == 1 ? dst : nullptr));
+            SDPA_TRY(run_fused(ctx, s, b, s.qc[b].as<float>(), bs, splits, part, splits == 1 ? dst : nullptr));
             SDPA_TRY(time_end(s, 1, s.s_compute));
             if (is_umma(ctx->prec)) SDPA_TRY(launch_attn_umma_twin(s.plan, b, bs, splits, part, splits == 1 ? dst : nullptr, s.s_compute));
             ++fused_launches;
@@ -1688,15 +1751,19 @@ static sdpa_status scatter_attention_impl(sdpa_ctx* ctx, const double* Q, const 
         set_error("attention(): bad dimensions or NULL input on rank 0 (m=%d n=%d dk=%d dv=%d)", m, n, dk, dv);
         return SDPA_ERR_INVALID;
     }
-    const int prec = resolve_precision(ctx->cfg.precision, dk, dv);
+    const int prec = resolve_precision(SDPA_DTYPE_F64, ctx->cfg.precision, dk, dv);
     SDPA_TRY(check_precision(prec, dk, dv));
     ctx->dk = dk;
     ctx->dv = dv;
     ctx->prec = prec;
+    ctx->dtype = SDPA_DTYPE_F64;
+    ctx->zero_copy = false;
     const size_t esz = elem_size(prec);
     s.n_local = sdpa_owner_count(n, ctx->world, s.grank);
     SDPA_TRY(s.Kc.reserve(((size_t)s.n_local + 128) * dk * esz));
     SDPA_TRY(s.Vc.reserve(((size_t)s.n_local + 128) * dv * esz));
+    s.k_in = s.Kc.p;
+    s.v_in = s.Vc.p;
     s.k_lo_off = ((size_t)s.n_local + 128) * dk;
     s.v_lo_off = ((size_t)s.n_local + 128) * dv;
     DevBuf sendbuf[2];
@@ -1755,8 +1822,13 @@ int sdpa_owner_disp(int n, int size, int rank)
 
 int sdpa_precision_supported(int precision, int dk, int dv, int* resolved)
 {
-    if (precision < SDPA_PREC_AUTO || precision > SDPA_PREC_BF16X3 || dk < 1 || dv < 1) return 0;
-    const int prec = resolve_precision(precision, dk, dv);
+    return sdpa_precision_supported_for(SDPA_DTYPE_F64, precision, dk, dv, resolved);
+}
+
+int sdpa_precision_supported_for(int dtype, int precision, int dk, int dv, int* resolved)
+{
+    if (!dtype_valid(dtype) || precision < SDPA_PREC_AUTO || precision > SDPA_PREC_BF16X3 || dk < 1 || dv < 1) return 0;
+    const int prec = resolve_precision(dtype, precision, dk, dv);
     if (resolved) *resolved = prec;
     if (is_umma(prec)) return attn_umma_supported(dk, dv, prec_hl(prec)) ? 1 : 0;
     return attn_f32_supported(dk, dv) ? 1 : 0;
@@ -1970,13 +2042,15 @@ sdpa_status sdpa_ctx_destroy(sdpa_ctx* ctx)
 sdpa_status sdpa_load_kv_host(sdpa_ctx* ctx, const double* const* K_shards, const double* const* V_shards,
                               const int* n_local, int dk, int dv)
 {
-    return load_kv(ctx, K_shards, V_shards, n_local, dk, dv, false);
+    return load_kv(ctx, SDPA_DTYPE_F64, reinterpret_cast<const void* const*>(K_shards), reinterpret_cast<const void* const*>(V_shards),
+                   n_local, dk, dv, false);
 }
 
 sdpa_status sdpa_load_kv_device(sdpa_ctx* ctx, const double* const* K_shards, const double* const* V_shards,
                                 const int* n_local, int dk, int dv)
 {
-    return load_kv(ctx, K_shards, V_shards, n_local, dk, dv, true);
+    return load_kv(ctx, SDPA_DTYPE_F64, reinterpret_cast<const void* const*>(K_shards), reinterpret_cast<const void* const*>(V_shards),
+                   n_local, dk, dv, true);
 }
 
 sdpa_status sdpa_load_kv_host_full(sdpa_ctx* ctx, const double* K, const double* V, int n, int dk, int dv)
@@ -1990,7 +2064,7 @@ sdpa_status sdpa_load_kv_host_full(sdpa_ctx* ctx, const double* K, const double*
         return SDPA_ERR_INVALID;
     }
     const int L = (int)ctx->shards.size();
-    std::vector<const double*> kp(L), vp(L);
+    std::vector<const void*> kp(L), vp(L);
     std::vector<int> cnt(L);
     // Distribution policy, the GPU analogue of the reference's Bcast-vs-Scatterv switch (mpi.c:213-215: K/V under 64 MiB
     // in fp32 are broadcast whole): with K/V replicated the Q rows can be sharded instead and no exchange is needed.
@@ -2003,7 +2077,7 @@ sdpa_status sdpa_load_kv_host_full(sdpa_ctx* ctx, const double* K, const double*
         kp[i] = K ? K + (size_t)d * dk : nullptr;
         vp[i] = V ? V + (size_t)d * dv : nullptr;
     }
-    SDPA_TRY(load_kv(ctx, kp.data(), vp.data(), cnt.data(), dk, dv, false));
+    SDPA_TRY(load_kv(ctx, SDPA_DTYPE_F64, kp.data(), vp.data(), cnt.data(), dk, dv, false));
     ctx->qshard = replicate;
     return SDPA_OK;
 }
@@ -2024,37 +2098,45 @@ sdpa_status sdpa_attention_device(sdpa_ctx* ctx, const double* const* Q_dev, dou
         set_error("sdpa_attention_device: the resident K/V is replicated (SDPA_DIST_Q); that distribution serves host arrays only");
         return SDPA_ERR_UNSUPPORTED;
     }
-    return attention_impl(ctx, nullptr, Q_dev, result_dev, true, m);
+    return attention_impl(ctx, nullptr, reinterpret_cast<const void* const*>(Q_dev), result_dev, true, m);
 }
 
-/* attention() on device-resident fp64 arrays in one call: K/V shard cast + Q batches + merge. */
-sdpa_status sdpa_attention_device_full(sdpa_ctx* ctx, const double* const* K_shards, const double* const* V_shards,
-                                       const int* n_local, int dk, int dv, const double* const* Q_dev, double* result_dev, int m)
+/* One pass on device-resident arrays of element type `dtype`: K/V shard cast (or none, where the fused kernel reads the arrays in
+ * place) + Q batches + merge.  blocking = false: queued (sdpa_enqueue_device_*), repaired at sdpa_synchronize. */
+static sdpa_status device_pass(sdpa_ctx* ctx, int dtype, const void* const* K_shards, const void* const* V_shards, const int* n_local,
+                               int dk, int dv, const void* const* Q_dev, void* result_dev, int m, bool blocking, const char* what)
 {
-    if (m > 0 && !Q_dev) {
-        set_error("sdpa_attention_device_full: Q_dev is NULL");
+    if (!dtype_valid(dtype)) {
+        set_error("%s: unknown dtype %d", what, dtype);
         return SDPA_ERR_INVALID;
     }
-    SDPA_TRY(load_kv(ctx, K_shards, V_shards, n_local, dk, dv, true, true));
-    return attention_impl(ctx, nullptr, Q_dev, result_dev, true, m);
-}
-
-/* The same pass, queued: returns as soon as the work is enqueued (stream order keeps consecutive passes and their
- * shared buffers in sequence); sdpa_synchronize() waits.  All arrays must stay valid until then. */
-sdpa_status sdpa_enqueue_device_full(sdpa_ctx* ctx, const double* const* K_shards, const double* const* V_shards,
-                                     const int* n_local, int dk, int dv, const double* const* Q_dev, double* result_dev, int m)
-{
     if (m > 0 && !Q_dev) {
-        set_error("sdpa_enqueue_device_full: Q_dev is NULL");
+        set_error("%s: Q_dev is NULL", what);
         return SDPA_ERR_INVALID;
     }
-    // Cast-ahead: where the persistent fused kernel takes the pass (it leaves room on every SM for one small CTA), on one GPU or
-    // with the overlapped device-side exchange, the casts of this pass run beside the previous pass's fused kernel.
+    const size_t esz = dtype_size(dtype);
+    if (ctx && n_local && dk >= 1 && dv >= 1) {
+        // Operands read in place: the tensor-core kernels load them through TMA, whose global addresses must be 16-byte aligned;
+        // the fp32 kernel takes any fp32 array.  A misaligned operand is refused, not copied.
+        const int prec = resolve_precision(dtype, ctx->cfg.precision, dk, dv);
+        const size_t align = is_umma(prec) ? 16 : esz;
+        auto bad = [&](const void* p) { return p && (uintptr_t)p % align != 0; };
+        for (size_t i = 0; i < ctx->shards.size() && reads_in_place(dtype, prec); ++i)
+            if ((n_local[i] > 0 && K_shards && V_shards && (bad(K_shards[i]) || bad(V_shards[i]))) || (m > 0 && bad(Q_dev[i]))) {
+                set_error("%s: %s operands are read in place by the %s kernel, which needs K, V and Q aligned to %zu bytes "
+                          "(shard %zu: K=%p V=%p Q=%p)", what, dtype_name(dtype), kernel_name(prec, dk, dv), align, i,
+                          K_shards ? K_shards[i] : nullptr, V_shards ? V_shards[i] : nullptr, m > 0 ? Q_dev[i] : nullptr);
+                return SDPA_ERR_INVALID;
+            }
+    }
+    // Cast-ahead (queued fp64 passes): where the persistent fused kernel takes the pass (it leaves room on every SM for one small
+    // CTA), on one GPU or with the overlapped device-side exchange, the casts of this pass run beside the previous pass's fused
+    // kernel.  Typed passes never cast ahead: they are "plain" queued passes (ev_plain_end).
     bool ahead = false;
-    if (ctx && ctx->cast_ahead && !ctx->repairing && n_local && m > 0 && dk == 128 && dv == 128) {
+    if (!blocking && dtype == SDPA_DTYPE_F64 && ctx && ctx->cast_ahead && !ctx->repairing && n_local && m > 0 && dk == 128 && dv == 128) {
         const int L = (int)ctx->shards.size();
         const bool ipc = ctx->world > 1 && ctx->cfg.merge == SDPA_MERGE_PEER && L == 1 && ctx->overlap_passes;
-        const int prec = resolve_precision(ctx->cfg.precision, dk, dv);
+        const int prec = resolve_precision(dtype, ctx->cfg.precision, dk, dv);
         // single-batch passes only: between two batches of one pass the side kernel would be released while other kernels
         // still run, and its CTAs pile up on the SMs that happen to have room (see the gate of the pushsync root form)
         const int B = pick_q_batch(ctx, m);
@@ -2068,20 +2150,22 @@ sdpa_status sdpa_enqueue_device_full(sdpa_ctx* ctx, const double* const* K_shard
             return false;
         };
         for (int i = 0; i < L && ahead; ++i)
-            if ((K_shards && aliases_result(K_shards[i], (size_t)n_local[i] * dk * sizeof(double))) ||
-                (V_shards && aliases_result(V_shards[i], (size_t)n_local[i] * dv * sizeof(double))) ||
-                aliases_result(Q_dev[i], (size_t)m * dk * sizeof(double)))
+            if ((K_shards && aliases_result(K_shards[i], (size_t)n_local[i] * dk * esz)) ||
+                (V_shards && aliases_result(V_shards[i], (size_t)n_local[i] * dv * esz)) ||
+                aliases_result(Q_dev[i], (size_t)m * dk * esz))
                 ahead = false;
     }
-    SDPA_TRY(load_kv(ctx, K_shards, V_shards, n_local, dk, dv, true, true, ahead));
-    SDPA_TRY(attention_impl(ctx, nullptr, Q_dev, result_dev, true, m, false, false));
+    SDPA_TRY(load_kv(ctx, dtype, K_shards, V_shards, n_local, dk, dv, true, true, ahead));
+    SDPA_TRY(attention_impl(ctx, nullptr, Q_dev, result_dev, true, m, false, blocking, dtype));
+    if (blocking) return SDPA_OK;
     if (result_dev && m > 0) {
         if (ctx->queued_results.size() >= 64) ctx->queued_results.erase(ctx->queued_results.begin());   // bounded: older ones are long complete
-        ctx->queued_results.push_back({reinterpret_cast<const char*>(result_dev), (size_t)m * dv * sizeof(double)});
+        ctx->queued_results.push_back({reinterpret_cast<const char*>(result_dev), (size_t)m * dv * esz});
     }
     if (ctx->deferring && !ctx->call_guards.empty()) {
         const size_t L = ctx->shards.size();
         sdpa_ctx::PendingPass p;
+        p.dtype = dtype;
         p.K.assign(K_shards, K_shards + L);
         p.V.assign(V_shards, V_shards + L);
         p.Q.assign(Q_dev, Q_dev + L);
@@ -2094,6 +2178,35 @@ sdpa_status sdpa_enqueue_device_full(sdpa_ctx* ctx, const double* const* K_shard
         ctx->pending.push_back(std::move(p));
     }
     return SDPA_OK;
+}
+
+/* attention() on device-resident fp64 arrays in one call: K/V shard cast + Q batches + merge. */
+sdpa_status sdpa_attention_device_full(sdpa_ctx* ctx, const double* const* K_shards, const double* const* V_shards,
+                                       const int* n_local, int dk, int dv, const double* const* Q_dev, double* result_dev, int m)
+{
+    return device_pass(ctx, SDPA_DTYPE_F64, reinterpret_cast<const void* const*>(K_shards), reinterpret_cast<const void* const*>(V_shards),
+                       n_local, dk, dv, reinterpret_cast<const void* const*>(Q_dev), result_dev, m, true, "sdpa_attention_device_full");
+}
+
+/* The same pass, queued: returns as soon as the work is enqueued (stream order keeps consecutive passes and their
+ * shared buffers in sequence); sdpa_synchronize() waits.  All arrays must stay valid until then. */
+sdpa_status sdpa_enqueue_device_full(sdpa_ctx* ctx, const double* const* K_shards, const double* const* V_shards,
+                                     const int* n_local, int dk, int dv, const double* const* Q_dev, double* result_dev, int m)
+{
+    return device_pass(ctx, SDPA_DTYPE_F64, reinterpret_cast<const void* const*>(K_shards), reinterpret_cast<const void* const*>(V_shards),
+                       n_local, dk, dv, reinterpret_cast<const void* const*>(Q_dev), result_dev, m, false, "sdpa_enqueue_device_full");
+}
+
+sdpa_status sdpa_attention_device_typed(sdpa_ctx* ctx, int dtype, const void* const* K_shards, const void* const* V_shards,
+                                        const int* n_local, int dk, int dv, const void* const* Q_dev, void* result_dev, int m)
+{
+    return device_pass(ctx, dtype, K_shards, V_shards, n_local, dk, dv, Q_dev, result_dev, m, true, "sdpa_attention_device_typed");
+}
+
+sdpa_status sdpa_enqueue_device_typed(sdpa_ctx* ctx, int dtype, const void* const* K_shards, const void* const* V_shards,
+                                      const int* n_local, int dk, int dv, const void* const* Q_dev, void* result_dev, int m)
+{
+    return device_pass(ctx, dtype, K_shards, V_shards, n_local, dk, dv, Q_dev, result_dev, m, false, "sdpa_enqueue_device_typed");
 }
 
 /* Deferred guard repair: wait for the queued passes, read the guard rings once, agree across processes, re-run (exact variant
@@ -2139,7 +2252,8 @@ static sdpa_status resolve_pending(sdpa_ctx* ctx)
     for (Shard& s : ctx->shards) umma_plan_force_exact(s.plan, true);
     sdpa_status st = SDPA_OK;
     for (sdpa_ctx::PendingPass& p : todo) {
-        st = sdpa_attention_device_full(ctx, p.K.data(), p.V.data(), p.n_local.data(), p.dk, p.dv, p.Q.data(), p.result, p.m);
+        st = device_pass(ctx, p.dtype, p.K.data(), p.V.data(), p.n_local.data(), p.dk, p.dv, p.Q.data(), p.result, p.m, true,
+                         "sdpa_synchronize (repair)");
         if (st != SDPA_OK) break;
     }
     for (Shard& s : ctx->shards) umma_plan_force_exact(s.plan, false);
@@ -2169,7 +2283,7 @@ sdpa_status sdpa_online_softmax_partials(sdpa_ctx* ctx, int local, const float* 
         set_error("sdpa_online_softmax_partials: bad arguments");
         return SDPA_ERR_INVALID;
     }
-    if (ctx->dk == 0 || ctx->prec != SDPA_PREC_F32) {
+    if (ctx->dk == 0 || ctx->prec != SDPA_PREC_F32 || ctx->zero_copy) {
         set_error("sdpa_online_softmax_partials needs a resident fp32 K/V shard (precision f32)");
         return SDPA_ERR_INVALID;
     }

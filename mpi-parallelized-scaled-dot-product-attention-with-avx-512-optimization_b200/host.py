@@ -32,6 +32,9 @@ PREC_AUTO, PREC_F32, PREC_BF16, PREC_BF16X3 = 0, 1, 2, 3
 MERGE_NCCL, MERGE_PEER, MERGE_NCCL2 = 0, 1, 2
 _MERGE = {"nccl": MERGE_NCCL2, "nccl2": MERGE_NCCL2, "nccl3": MERGE_NCCL, "peer": MERGE_PEER}
 DIST_KV, DIST_Q, DIST_AUTO = 0, 1, 2
+DTYPE_F64, DTYPE_F32, DTYPE_BF16 = 0, 1, 2
+_DTYPE = {"f64": DTYPE_F64, "fp64": DTYPE_F64, "float64": DTYPE_F64, "f32": DTYPE_F32, "fp32": DTYPE_F32, "float32": DTYPE_F32,
+          "bf16": DTYPE_BF16, "bfloat16": DTYPE_BF16}
 _DIST = {"kv": DIST_KV, "q": DIST_Q, "auto": DIST_AUTO}
 _PREC = {"auto": PREC_AUTO, "f32": PREC_F32, "fp32": PREC_F32, "bf16": PREC_BF16, "bf16x3": PREC_BF16X3, "f32x3": PREC_BF16X3}
 
@@ -70,6 +73,7 @@ ABI = {
     "sdpa_owner_count": (ctypes.c_int, [ctypes.c_int] * 3),
     "sdpa_owner_disp": (ctypes.c_int, [ctypes.c_int] * 3),
     "sdpa_precision_supported": (ctypes.c_int, [ctypes.c_int] * 3 + [ctypes.POINTER(ctypes.c_int)]),
+    "sdpa_precision_supported_for": (ctypes.c_int, [ctypes.c_int] * 4 + [ctypes.POINTER(ctypes.c_int)]),
     "sdpa_config_init": (None, [ctypes.POINTER(Config)]),
     "sdpa_ctx_create": (ctypes.c_int, [ctypes.POINTER(_V), ctypes.POINTER(Config), _V]),
     "sdpa_ctx_destroy": (ctypes.c_int, [_V]),
@@ -86,6 +90,8 @@ ABI = {
     "sdpa_host_copy": (ctypes.c_int, [_V, _V, ctypes.c_size_t]),
     "sdpa_enqueue_device_full": (ctypes.c_int, [_V, _dpp, _dpp, _ip, ctypes.c_int, ctypes.c_int, _dpp, _V, ctypes.c_int]),
     "sdpa_synchronize": (ctypes.c_int, [_V]),
+    "sdpa_attention_device_typed": (ctypes.c_int, [_V, ctypes.c_int, _dpp, _dpp, _ip, ctypes.c_int, ctypes.c_int, _dpp, _V, ctypes.c_int]),
+    "sdpa_enqueue_device_typed": (ctypes.c_int, [_V, ctypes.c_int, _dpp, _dpp, _ip, ctypes.c_int, ctypes.c_int, _dpp, _V, ctypes.c_int]),
     "sdpa_scatter_attention": (ctypes.c_int, [_V, _V, _V, _V, _V] + [ctypes.c_int] * 4),
     "sdpa_online_softmax_partials": (ctypes.c_int, [_V, ctypes.c_int, _V, ctypes.c_int, _V, _V, _V]),
     "sdpa_last_timings": (ctypes.c_int, [_V, _fp]),
@@ -192,6 +198,23 @@ def precision_supported(precision, dk: int, dv: int):
     """(supported, resolved precision name) -- which kernel family a (precision, dk, dv) request lands on."""
     res = ctypes.c_int(-1)
     ok = lib().sdpa_precision_supported(_PREC[precision] if isinstance(precision, str) else int(precision), dk, dv, ctypes.byref(res))
+    names = {PREC_F32: "f32", PREC_BF16: "bf16", PREC_BF16X3: "bf16x3"}
+    return bool(ok), names.get(res.value)
+
+
+def _dtype(dtype) -> int:
+    """An sdpa_dtype from a name ("bf16", "fp32", ...), a torch / NumPy dtype, or the integer itself."""
+    if isinstance(dtype, int):
+        return dtype
+    return _DTYPE[str(dtype).rsplit(".", 1)[-1]]
+
+
+def precision_supported_for(dtype, precision, dk: int, dv: int):
+    """:func:`precision_supported` for operands of element type ``dtype``: bf16 operands resolve AUTO to the bf16 kernel
+    (where it takes the shape), fp64 / fp32 operands follow the fp64 rule."""
+    res = ctypes.c_int(-1)
+    ok = lib().sdpa_precision_supported_for(_dtype(dtype), _PREC[precision] if isinstance(precision, str) else int(precision), dk, dv,
+                                             ctypes.byref(res))
     names = {PREC_F32: "f32", PREC_BF16: "bf16", PREC_BF16X3: "bf16x3"}
     return bool(ok), names.get(res.value)
 
@@ -331,6 +354,18 @@ class Context:
         fn = lib().sdpa_attention_device_full if blocking else lib().sdpa_enqueue_device_full
         _check(fn(self._h, ka, va, counts, dk, dv, qa, ctypes.c_void_p(result_ptr or 0), m),
                "sdpa_attention_device_full" if blocking else "sdpa_enqueue_device_full")
+        self.dk, self.dv = dk, dv
+
+    def attention_device_typed(self, dtype, K_ptrs, V_ptrs, n_local, dk: int, dv: int, Q_ptrs, result_ptr: int | None, m: int,
+                               blocking: bool = True) -> None:
+        """:meth:`attention_device_full` on device arrays of element type ``dtype`` ("f64", "f32", "bf16", a torch dtype or
+        ``DTYPE_*``); the result has the same type.  bf16 operands at the bf16 kernel and fp32 operands at the fp32 kernel are
+        read in place (no cast kernel runs)."""
+        counts = (ctypes.c_int * self.num_local)(*[int(c) for c in n_local])
+        fn = lib().sdpa_attention_device_typed if blocking else lib().sdpa_enqueue_device_typed
+        _check(fn(self._h, _dtype(dtype), self._ptr_array(K_ptrs), self._ptr_array(V_ptrs), counts, dk, dv, self._ptr_array(Q_ptrs),
+                  ctypes.c_void_p(result_ptr or 0), m),
+               "sdpa_attention_device_typed" if blocking else "sdpa_enqueue_device_typed")
         self.dk, self.dv = dk, dv
 
     def synchronize(self) -> None:
